@@ -329,6 +329,21 @@ def step_bytes_of(cfg, weight_bytes, B, ctx):
     return weight_bytes + B * ctx * cfg["num_layers"] * 2 * cfg["num_kv_heads"] * cfg["dim_head"] * 2
 
 
+DUMP_LOGITS_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, tokens, logits):
+    """What the caller of the timed step receives: the greedy picks, and the logits they were picked from.  Inputs are
+    seeded, so two builds can be compared array by array; logits larger than DUMP_LOGITS_BYTES keep a fixed sample of rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "next_tokens.npy"), tokens.astype(np.float64))
+    if logits.nbytes > DUMP_LOGITS_BYTES:
+        rows = np.sort(np.random.RandomState(0).choice(logits.shape[0], DUMP_LOGITS_BYTES // logits[0].nbytes, replace=False))
+        logits = logits[rows]
+    np.save(os.path.join(out_dir, "logits.npy"), logits.astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -351,6 +366,9 @@ def main():
                     help="default: the model's BASELINE quantisation (GPTQ int4 for 8B, bf16 for 1B); int8 / fp8: W8A8 Linear rows")
     ap.add_argument("--prefill-chunk", type=int, default=128, help="tokens per chunked-prefill pass of the TTFT measurement")
     ap.add_argument("--fuse", type=int, default=2, help="0: one kernel per reference op; 1: +RMSNorm fused; 2: +qkv RoPE/KV epilogue")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/next_tokens.npy (B) and DIR/logits.npy (B, vocab/N of "
+                         "rank 0; a fixed sample of rows above %d MB), float64 / float32" % (DUMP_LOGITS_BYTES >> 20))
     args = ap.parse_args()
 
     cfg = model_cfg(args.model)
@@ -419,6 +437,8 @@ def main():
     launches0 = dec.lib.zl_launch_count(0)
     ms_dev, clocks = measure_decode(dec, B, args.steps, W, stream, barrier, sampler_gpu=local_rank)
     weight_bytes, kernels_per_step = dec.stats(B)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dec.get_state(B)[0], dec.logits(B))
 
     # sanity of the synthetic model: the logits of the last timed step must be finite (a NaN step costs the same time)
     tok, pos = dec.get_state(B)

@@ -380,6 +380,8 @@ int zl_llama_set_state(zl_llama_t* m, const int32_t* tokens_host, const int32_t*
 int zl_llama_step_device(zl_llama_t* m, int B);
 /* read back the device-resident (token, position) state; synchronous. */
 int zl_llama_get_state(zl_llama_t* m, int32_t* tokens_host, int32_t* positions_host, int B);
+/* read back the fp32 logits (B, vocab/tp) of the most recent decode step (this rank's shard); synchronous. */
+int zl_llama_get_logits(zl_llama_t* m, float* logits_host, int B);
 int zl_llama_sync(zl_llama_t* m);
 /* Chunked prefill of ONE task (SearchTask prompt, src/generator/batch_generator.cpp:1576): appends tokens_host[0..n) at
  * positions pos0.. to the task's KV buffers through the same kernels (M = chunk GEMMs, causal len_q = chunk attention)

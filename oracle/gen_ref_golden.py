@@ -378,7 +378,9 @@ def main(out_dir, lib_path=None):
         kq.append(a.view(k.shape)); sk.append(s.view(k.shape[0], c["hkv"]))
         b, s2 = ref.quant_u8(ref.t(v.reshape(-1, c["d"])))
         vq.append(b.view(v.shape)); sv.append(s2.view(v.shape[0], c["hkv"]))
-        outs["kq%d" % i], outs["sk%d" % i], outs["vq%d" % i], outs["sv%d" % i] = n(kq[-1]), n(sk[-1]), n(vq[-1]), n(sv[-1])
+        # the uint8 codes as digests: the whole cache would make the fixture larger than 1 MB
+        outs["kq%d_digest" % i], outs["vq%d_digest" % i] = np.array(gc.digest(n(kq[-1]))), np.array(gc.digest(n(vq[-1])))
+        outs["sk%d" % i], outs["sv%d" % i] = n(sk[-1]), n(sv[-1])
     mask = ref.t(np.concatenate([m.reshape(-1) for m in c["masks"]]))
     outs["out"] = n(ref.attention_kv8(ref.t(c["q"]), ref.t(c["lens"]), kq, vq, sk, sv, mask, c["scale"], c["hkv"]).float())
     np.savez(os.path.join(out_dir, "ref_kv8.npz"), **outs)

@@ -1,7 +1,7 @@
 """Shared test helpers (numpy restatement of OUR ZLW4 tile layout + small utilities)."""
 import numpy as np
 
-from oracle import gptq
+from oracle import golden_cases, gptq
 
 BLK = 2128
 
@@ -55,6 +55,22 @@ def rel_l2(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)
     return float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-30))
+
+
+def tensor_digest(t):
+    """golden_cases.digest of a torch tensor (bf16 hashed as its 16-bit patterns)."""
+    import torch
+    t = t.detach().contiguous().cpu()
+    if t.dtype == torch.bfloat16:
+        t = t.view(torch.int16)
+    return golden_cases.digest(t.numpy())
+
+
+def sample_index(size, n):
+    """A fixed, seeded choice of n of `size` flat indices (all of them when n >= size)."""
+    if n >= size:
+        return np.arange(size)
+    return np.sort(np.random.RandomState(0).choice(size, n, replace=False))
 
 
 def to_bf16_bits(x):

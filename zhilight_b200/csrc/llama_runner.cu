@@ -1345,6 +1345,17 @@ extern "C" int zl_llama_get_state(zl_llama_t* m, int32_t* tokens_host, int32_t* 
     return ZL_OK;
 }
 
+extern "C" int zl_llama_get_logits(zl_llama_t* m, float* logits_host, int B) {
+    ZL_CHECK_ARG(m && logits_host && B > 0 && B <= m->cfg.max_batch);
+    if (!m->finalized) {
+        zl_set_last_error(__FILE__, __LINE__, "model not finalized");
+        return ZL_ERR_STATE;
+    }
+    ZL_CHECK_CUDA(cudaMemcpyAsync(logits_host, m->logits, (size_t)B * m->vshard * 4, cudaMemcpyDeviceToHost, m->stream));
+    ZL_CHECK_CUDA(cudaStreamSynchronize(m->stream));
+    return ZL_OK;
+}
+
 extern "C" int zl_llama_bench_gemms(zl_llama_t* m, int B, int iters, float* ms, int* launches, double* bytes) {
     ZL_CHECK_ARG(m && B > 0 && B <= m->cfg.max_batch && iters > 0 && ms);
     const auto& c = m->cfg;

@@ -117,6 +117,12 @@ class LlamaDecoder:
                                                p.ctypes.data_as(ctypes.c_void_p), b))
         return t, p
 
+    def logits(self, b):
+        """fp32 logits (B, V/tp) of the most recent step: this rank's vocabulary shard."""
+        out = np.empty((b, self.vocab_shard), dtype=np.float32)
+        _lib.check(self.lib.zl_llama_get_logits(self.h, out.ctypes.data_as(ctypes.c_void_p), b))
+        return out
+
     def step_device(self, b):
         _lib.check(self.lib.zl_llama_step_device(self.h, b))
 
