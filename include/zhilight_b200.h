@@ -246,6 +246,11 @@ int zl_qkv_rope_append(const float* cos, const float* sin, const void* qkv, void
  * (weights of a later GEMM; attention leaves HBM idle at small batch). */
 int zl_decode_attention_set_prefetch(const void* ptr, size_t bytes);
 size_t zl_decode_attention_workspace_bytes(int B, int len_q, int num_heads, int dim_head, int max_len_buf);
+/* tests: host view of the launch zl_decode_attention makes for this shape (the same code chooses it): *kernel = 0
+ * k_decode_attn (P.V on the tensor cores), 1 warp-per-32-keys kernel, 2 / 3 the ZL_ATTN_OLD_SHORT / ZL_ATTN_PV_FP32
+ * variants; *splits = KV splits, each CTA covering round16(ceil(len_buf / splits)) keys of its task. */
+int zl_decode_attention_plan(int B, int len_q, int num_heads, int num_kv_heads, int max_len_buf, int* kernel,
+                             int* splits);
 /* q (B, len_q, H_q, d); buf_lens (B); k_addrs/v_addrs (B) device arrays of device pointers;
  * mask int8 ragged concat of (len_q, len_buf_b); out (B, len_q, H_q, d).  bshd: (len_buf, H_kv, d) else
  * (H_kv, len_buf, d). */

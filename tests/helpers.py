@@ -51,6 +51,14 @@ def w4_pack_numpy(qw_km, qz_km, sc_km, sym=False, row_map=None):
     return out.reshape(-1)
 
 
+def attention_plan(lib, b, len_q, hq, hkv, max_len):
+    """(kernel, splits) that zl_decode_attention launches for this shape: kernel 0 = k_decode_attn, 1 = warp kernel"""
+    import ctypes
+    kernel, splits = ctypes.c_int(-1), ctypes.c_int(-1)
+    assert lib.zl_decode_attention_plan(b, len_q, hq, hkv, max_len, ctypes.byref(kernel), ctypes.byref(splits)) == 0
+    return kernel.value, splits.value
+
+
 def rel_l2(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)

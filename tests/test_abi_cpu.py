@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+from tests.helpers import attention_plan
 from zhilight_b200 import _lib
 
 
@@ -103,3 +104,40 @@ def test_tcgen05_stream_k_schedule_covers_every_unit_once(n_tiles, G, ctas):
         assert all(p[2] == len(ps) for p in ps), (tile, ps)
         assert ps[0][0] == 0 and ps[-1][1] == G and all(a[1] == b[0] for a, b in zip(ps, ps[1:]))
         assert [p[3] for p in ps] == list(range(ps[0][3], ps[0][3] + len(ps))), "pieces in k order belong to consecutive CTAs"
+
+
+def test_decode_attention_plan_fits_every_kernel(lib):
+    """zl_decode_attention_plan is the launch decision of zl_decode_attention.  Both kernels size their shared memory for a
+    fixed number of keys per CTA and trust the host to keep round16(ceil(len_buf / splits)) within it: 256 for the
+    warp-per-32-keys kernel, 1024 for k_decode_attn.  The splits must also cover the context and fit the workspace that
+    zl_decode_attention_workspace_bytes reports."""
+    d = 128
+    heads = [(8, 8), (32, 8), (40, 8), (28, 4), (64, 8), (48, 4), (32, 2)]      # m_query 1, 4, 5, 7, 8, 12, 16
+    lens = [1, 15, 16, 17, 255, 256, 257, 1023, 1024, 1025, 16384, 16385, 65536, 70000, 131072]
+    max_keys = {0: 1024, 1: 256}
+    for b in range(1, 65):
+        for len_q in (1, 3, 64, 128):
+            for hq, hkv in heads:
+                for max_len in lens:
+                    kernel, splits = attention_plan(lib, b, len_q, hq, hkv, max_len)
+                    case = (b, len_q, hq, hkv, max_len, kernel, splits)
+                    assert kernel in max_keys and splits >= 1, case
+                    chunk = (-(-max_len // splits) + 15) // 16 * 16
+                    assert chunk <= max_keys[kernel], case
+                    assert splits * chunk >= max_len, case
+                    if splits > 1:
+                        need = b * len_q * hq * splits * (d + 2) * 4
+                        assert lib.zl_decode_attention_workspace_bytes(b, len_q, hq, d, max_len) >= need, case
+
+
+@pytest.mark.parametrize("b,len_q,max_len,splits", [
+    (1, 128, 128, 1), (1, 128, 256, 1),              # 8B prefill, chunk 128: both chunks of a 256-token prompt
+    (32, 1, 2048, 2),                                # batch 32 decode at context 2048
+    (8, 1, 8192, 8),                                 # batch 8, context 8192
+    (1, 1, 20000, 37), (1, 1, 70000, 69),            # batch 1, long context (more splits than a short context allows)
+    (32, 1, 513, 2), (32, 1, 4096, 4)])              # batch 32 decode past 512 tokens
+def test_decode_attention_plan_of_benchmarked_shapes(lib, b, len_q, max_len, splits):
+    """The shapes the project reports numbers for (Llama-3.1-8B heads, 32 / 8) run on k_decode_attn (kernel 0)."""
+    assert attention_plan(lib, b, len_q, 32, 8, max_len) == (0, splits)
+    bad = ctypes.c_int()
+    assert lib.zl_decode_attention_plan(b, len_q, 32, 7, max_len, ctypes.byref(bad), ctypes.byref(bad)) == -1

@@ -296,3 +296,34 @@ def test_large_batch_decode_on_8b_shapes_matches_batch_1(lib, cuda, b, graph, pd
         assert np.isfinite(lb).all(), step
         for t in (0, b // 2, b - 1):
             assert rel_l2(lb[t], l1[0]) <= 5e-3, (step, t)
+
+
+def test_prefill_chunk_128_on_8b_shapes_matches_decode_steps(lib, cuda, monkeypatch):
+    """The TTFT path on Llama-3.1-8B layer shapes: a 256-token prompt in two 128-token chunks (M = 128 GEMMs, causal
+    len_q = 128 attention on k_decode_attn) must leave the same KV state and last-position logits as 256 batch-1 decode
+    steps of the same tokens, and three decode steps from either state must agree."""
+    from zhilight_b200.llama import LlamaDecoder
+    from tests.helpers import attention_plan
+    cfg = LAYERS8B_SMALLV
+    monkeypatch.delenv("ZL_PREFILL_DUAL", raising=False)       # single-stream chunks: len_q = 128 per attention call
+    for keys in (128, 256):
+        assert attention_plan(lib, 1, 128, cfg["num_heads"], cfg["num_kv_heads"], keys)[0] == 0
+    prompt = np.random.default_rng(12).integers(0, cfg["vocab_size"], size=256).astype(np.int32)
+    pre = LlamaDecoder(quant_type=5, group_size=128, sym=True, max_batch=1, max_seq=512, prefill_chunk=128, **cfg)
+    pre.init_synthetic(seed=3)
+    _, lp = pre.prefill(0, prompt, want_logits=True)
+    dec = LlamaDecoder(quant_type=5, group_size=128, sym=True, max_batch=1, max_seq=512, **cfg)
+    dec.init_synthetic(seed=3)
+    for p, t in enumerate(prompt):
+        _, ld = dec.decode(np.array([t], np.int32), np.array([p], np.int32), want_logits=True)
+    assert np.isfinite(lp).all() and np.isfinite(ld).all()
+    assert rel_l2(lp, ld) <= 5e-3
+    tok, pos = np.array([int(np.argmax(ld[0]))], np.int32), np.array([len(prompt)], np.int32)
+    for step in range(3):
+        _, lp = pre.decode(tok, pos, want_logits=True)
+        nd, ld = dec.decode(tok, pos, want_logits=True)
+        assert np.isfinite(lp).all()
+        assert rel_l2(lp, ld) <= 5e-3, step
+        tok, pos = nd, pos + 1
+    pre.close()
+    dec.close()

@@ -24,6 +24,11 @@ constexpr int kAttnWarps = 4;
 constexpr int kAttnMaxRange = 1024;            // keys per CTA; logits live in shared memory
 constexpr int kAttnRowStride = kAttnMaxRange + 4;
 constexpr int kAttnMaxSplits = 64;
+// kernel ids reported by zl_decode_attention_plan
+constexpr int kAttnKernelTc = 0;               // k_decode_attn, P.V on the tensor cores
+constexpr int kAttnKernelWarp = 1;             // k_decode_attn_warp
+constexpr int kAttnKernelShort = 2;            // k_decode_attn_short (ZL_ATTN_OLD_SHORT)
+constexpr int kAttnKernelPvFp32 = 3;           // k_decode_attn, P.V on the CUDA cores (ZL_ATTN_PV_FP32)
 
 template <typename T, int D, bool PV_FP32>
 __global__ void __launch_bounds__(kAttnThreads)
@@ -368,6 +373,30 @@ extern "C" size_t zl_decode_attention_workspace_bytes(int B, int len_q, int num_
     return (size_t)B * len_q * num_heads * splits * (dim_head + 2) * sizeof(float);
 }
 
+extern "C" int zl_decode_attention_plan(int B, int len_q, int num_heads, int num_kv_heads, int max_len_buf, int* kernel,
+                                        int* splits) {
+    ZL_CHECK_ARG(kernel && splits && B > 0 && len_q > 0 && max_len_buf > 0);
+    ZL_CHECK_ARG(num_heads > 0 && num_kv_heads > 0 && num_heads % num_kv_heads == 0);
+    const int m_query = num_heads / num_kv_heads;
+    // latency regime: few CTAs of work -> 256-key CTAs that issue all their loads up front
+    const int hgroups = (m_query + 7) / 8;
+    const int short_splits = cdiv(max_len_buf, kShortRange);
+    const bool use_short = short_splits <= kAttnMaxSplits &&
+                           (long long)B * len_q * num_kv_heads * hgroups * short_splits <= 4 * 148;
+    // default for the latency regime: the warp-per-32-keys kernel (one __syncthreads per CTA); ZL_ATTN_OLD_SHORT=1 keeps the
+    // previous 512-thread short kernel and ZL_ATTN_PV_FP32=1 the CUDA-core P.V loop of k_decode_attn, for A/B measurements
+    static const bool old_short = getenv("ZL_ATTN_OLD_SHORT") != nullptr;
+    static const bool pv_fp32 = getenv("ZL_ATTN_PV_FP32") != nullptr;
+    if (use_short) {
+        *kernel = old_short ? kAttnKernelShort : kAttnKernelWarp;
+        *splits = short_splits;
+    } else {
+        *kernel = pv_fp32 ? kAttnKernelPvFp32 : kAttnKernelTc;
+        *splits = attn_num_splits(B, len_q, num_kv_heads, m_query, max_len_buf);
+    }
+    return ZL_OK;
+}
+
 extern "C" int zl_decode_attention(const void* q, const int32_t* buf_lens, void* const* k_addrs,
                                    void* const* v_addrs, const int8_t* mask, float scale, int max_len_buf,
                                    void* out, int B, int len_q, int num_heads, int num_kv_heads, int dim_head,
@@ -378,13 +407,9 @@ extern "C" int zl_decode_attention(const void* q, const int32_t* buf_lens, void*
     ZL_CHECK_SUPPORTED(dim_head == 64 || dim_head == 128);
     ZL_CHECK_SUPPORTED(dtype == ZL_F16 || dtype == ZL_BF16);
     const int m_query = num_heads / num_kv_heads;
-    int splits = attn_num_splits(B, len_q, num_kv_heads, m_query, max_len_buf);
-    // latency regime: few CTAs of work -> 256-key CTAs that issue all their loads up front
-    const int hg0 = (m_query + 7) / 8;
-    const int short_splits = cdiv(max_len_buf, kShortRange);
-    const bool use_short = short_splits <= kAttnMaxSplits &&
-                           (long long)B * len_q * num_kv_heads * hg0 * short_splits <= 4 * 148;
-    if (use_short) splits = short_splits;
+    int kernel = 0, splits = 0;
+    const int rc = zl_decode_attention_plan(B, len_q, num_heads, num_kv_heads, max_len_buf, &kernel, &splits);
+    if (rc != ZL_OK) return rc;
     const size_t vheads = (size_t)B * len_q * num_heads;
     float* part_o = nullptr;
     float* part_m = nullptr;
@@ -398,18 +423,13 @@ extern "C" int zl_decode_attention(const void* q, const int32_t* buf_lens, void*
     }
     const int hgroups = (m_query + 7) / 8;
     dim3 grid(splits, num_kv_heads * hgroups, B * len_q), block(kAttnThreads);
-    // default for the latency regime: the warp-per-32-keys kernel (one __syncthreads per CTA); ZL_ATTN_OLD_SHORT=1 keeps the
-    // previous 512-thread short kernel for A/B measurements
-    static const bool old_short = getenv("ZL_ATTN_OLD_SHORT") != nullptr;
-    static const bool pv_fp32 = getenv("ZL_ATTN_PV_FP32") != nullptr;
-    const bool use_warp = use_short && !old_short;
 #define ZL_ATTN_LAUNCH(TT, DD)                                                                                  \
-    if (use_warp) {                                                                                             \
+    if (kernel == kAttnKernelWarp) {                                                                            \
         ZL_CHECK_CUDA(launch(k_decode_attn_warp<TT, DD>, grid, dim3(kWarpAttnWarps * 32),                       \
                              (size_t)warp_attn_smem_floats<DD>() * sizeof(float), stream, pdl != 0, (const TT*)q, \
                              buf_lens, (TT* const*)k_addrs, (TT* const*)v_addrs, mask, scale, (TT*)out, part_o, \
                              part_m, part_l, len_q, num_heads, num_kv_heads, m_query, splits, bshd));            \
-    } else if (use_short) {                                                                                     \
+    } else if (kernel == kAttnKernelShort) {                                                                    \
         static bool attr_set = false;                                                                           \
         if (!attr_set) {                                                                                        \
             ZL_CHECK_CUDA(cudaFuncSetAttribute(k_decode_attn_short<TT, DD>,                                     \
@@ -422,7 +442,7 @@ extern "C" int zl_decode_attention(const void* q, const int32_t* buf_lens, void*
                              (TT* const*)v_addrs, mask, scale, (TT*)out, part_o, part_m, part_l, len_q,         \
                              num_heads, num_kv_heads, m_query, splits, bshd, g_attn_pf_ptr, g_attn_pf_bytes));                                  \
     } else                                                                                                      \
-    if (pv_fp32) {                                                                                              \
+    if (kernel == kAttnKernelPvFp32) {                                                                          \
         ZL_CHECK_CUDA(launch(k_decode_attn<TT, DD, true>, grid, block, 0, stream, pdl != 0, (const TT*)q, buf_lens, \
                              (TT* const*)k_addrs, (TT* const*)v_addrs, mask, scale, (TT*)out, part_o, part_m,   \
                              part_l, len_q, num_heads, num_kv_heads, m_query, splits, bshd, g_attn_pf_ptr,      \

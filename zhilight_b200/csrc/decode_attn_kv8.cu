@@ -55,6 +55,7 @@ k_decode_attn_kv8(const __half* __restrict__ q, const int32_t* __restrict__ buf_
     constexpr int NSUB = kA8Threads / DC;
     __shared__ __align__(16) float s_logit[8 * kA8RowStride];
     __shared__ float s_m[8], s_l[8];
+    __shared__ int s_wexp;                     // binary exponent of the largest V scale of the CTA's keys
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int g = lane >> 2, t = lane & 3;
@@ -140,22 +141,32 @@ k_decode_attn_kv8(const __half* __restrict__ q, const int32_t* __restrict__ buf_
         float mx = -1e20f;
         for (int i = lane; i < n; i += 32) mx = fmaxf(mx, row[i]);
         mx = warp_max(mx);
-        float sum = 0.f;
+        float sum = 0.f, svmax = 0.f;
         for (int i = lane; i < n; i += 32) {
             const float e = expf(row[i] - mx);
+            const float sv = __ldcg(svb + (size_t)(k0 + i) * num_kv_heads);
             sum += e;
-            row[i] = e * __ldcg(svb + (size_t)(k0 + i) * num_kv_heads);
+            svmax = fmaxf(svmax, fabsf(sv));
+            row[i] = e * sv;
         }
         sum = warp_sum(sum) + 1e-20f;
+        svmax = warp_max(svmax);
         if (lane == 0) {
             s_m[h] = mx;
             s_l[h] = sum;
+            if (h == 0) {
+                int ex;
+                frexpf(svmax, &ex);                  // svmax = m 2^ex, m in [0.5, 1)  (svmax = 0: ex = 0)
+                s_wexp = max(ex, -116);              // keeps 2^(10 - ex) and 2^(ex - 10) normal floats
+            }
         }
     }
     __syncthreads();
 
     // ---- phase 3: O = (P * scale_v) . (V - 128) on the tensor cores (mma.sync m16n8k16, fp32 accumulate) ----
-    // A = weights [head (8 of 16 rows) x 16 keys] as fp16 (scaled by 2^10 so that small probabilities stay normal numbers),
+    // A = weights [head (8 of 16 rows) x 16 keys] as fp16, scaled by 2^(10 - ex) where 2^ex bounds the largest V scale of the
+    // CTA's keys: every weight is p * scale_v <= scale_v, so the largest lands below 1024 (no fp16 overflow for any V
+    // magnitude) and near it (small weights stay normal numbers); the power of two is undone exactly at write-out.
     // B = V [16 keys x 8 columns] as exact fp16 integers.  A B fragment register holds TWO KEYS of one column, V is stored
     // key-major: lane (g, t) loads D/8 contiguous bytes (columns NJ g .. NJ g + NJ - 1) of its four keys 2t, 2t+1, 2t+8,
     // 2t+9 and byte-interleaves row pairs with PRMT; n-tile j column c then stands for column d = NJ c + j of V (any
@@ -166,6 +177,7 @@ k_decode_attn_kv8(const __half* __restrict__ q, const int32_t* __restrict__ buf_
 #pragma unroll
     for (int j = 0; j < NJ; ++j) o[j][0] = o[j][1] = o[j][2] = o[j][3] = 0.f;
     const __half2 voff = __float2half2_rn(1152.f);   // 1024 (magic) + 128 (zero point of the cache)
+    const float wscale = ldexpf(1.f, 10 - s_wexp);
     for (int tile = warp; tile < ntiles; tile += kA8Warps) {
         const int kb = tile * 16;                    // first key of the tile, relative to k0
         uint32_t vw[4][NW];
@@ -190,8 +202,8 @@ k_decode_attn_kv8(const __half* __restrict__ q, const int32_t* __restrict__ buf_
             const float* pr = s_logit + g * kA8RowStride + kb + 2 * t;
             const float2 p0 = *reinterpret_cast<const float2*>(pr), p1 = *reinterpret_cast<const float2*>(pr + 8);
             const bool in0 = kb + 2 * t < n, in1 = kb + 2 * t + 1 < n, in2 = kb + 2 * t + 8 < n, in3 = kb + 2 * t + 9 < n;
-            const __half2 h0 = __floats2half2_rn(in0 ? p0.x * 1024.f : 0.f, in1 ? p0.y * 1024.f : 0.f);
-            const __half2 h1 = __floats2half2_rn(in2 ? p1.x * 1024.f : 0.f, in3 ? p1.y * 1024.f : 0.f);
+            const __half2 h0 = __floats2half2_rn(in0 ? p0.x * wscale : 0.f, in1 ? p0.y * wscale : 0.f);
+            const __half2 h1 = __floats2half2_rn(in2 ? p1.x * wscale : 0.f, in3 ? p1.y * wscale : 0.f);
             af[0] = *reinterpret_cast<const uint32_t*>(&h0);   // (head g, keys 2t, 2t+1)
             af[2] = *reinterpret_cast<const uint32_t*>(&h1);   // (head g, keys 2t+8, 2t+9); rows g+8 (a1, a3) stay zero
         }
@@ -214,10 +226,11 @@ k_decode_attn_kv8(const __half* __restrict__ q, const int32_t* __restrict__ buf_
     float* s_red = s_logit;   // [warp][h][D]
     if (g < mq) {
         // accumulator (n-tile j, column c = 2t + i) = head g, V column NJ c + j; rows g + 8 (o[j][2..3]) are padding
+        const float wunscale = ldexpf(1.f, s_wexp - 10);
 #pragma unroll
         for (int j = 0; j < NJ; ++j) {
-            s_red[(warp * 8 + g) * D + NJ * (2 * t) + j] = o[j][0] * (1.f / 1024.f);
-            s_red[(warp * 8 + g) * D + NJ * (2 * t + 1) + j] = o[j][1] * (1.f / 1024.f);
+            s_red[(warp * 8 + g) * D + NJ * (2 * t) + j] = o[j][0] * wunscale;
+            s_red[(warp * 8 + g) * D + NJ * (2 * t + 1) + j] = o[j][1] * wunscale;
         }
     }
     __syncthreads();
@@ -356,10 +369,9 @@ extern "C" int zl_decode_attention_kv8(const void* q, const int32_t* buf_lens, v
     const int max_useful = cdiv(max_len_buf, 256);
     if (splits > max_useful) splits = max_useful;
     if (splits > kA8MaxSplits) splits = kA8MaxSplits;
-    const int min_splits = cdiv(max_len_buf, kA8MaxRange);
+    const int min_splits = cdiv(max_len_buf, kA8MaxRange);   // a CTA holds at most 1024 logits: may exceed kA8MaxSplits
     if (splits < min_splits) splits = min_splits;
     if (splits < 1) splits = 1;
-    ZL_CHECK_SUPPORTED(splits <= kA8MaxSplits);
     const size_t vheads = (size_t)B * len_q * num_heads;
     float *part_o = nullptr, *part_m = nullptr, *part_l = nullptr;
     if (splits > 1) {
