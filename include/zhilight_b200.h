@@ -294,6 +294,31 @@ int zl_argmax(const float* logits, int32_t* out, int T, int V, void* workspace, 
 int zl_argmax_candidates(const float* logits, void* cand_out, int T, int V, int idx_offset, void* workspace,
                          size_t workspace_bytes, int pdl, zl_stream_t stream);
 int zl_argmax_merge(const void* cand_all, int32_t* out, int T, int ranks, int stride, int pdl, zl_stream_t stream);
+/* Seeded sampling pick over fp32 logits (T, V), one launch for all rows.  Row b belongs to task row_task[b] (device
+ * int32, each task at most once per call) whose parameters are params[task] (device array):
+ *   penalties on every token t set in the task's seen bits (uint32[ceil(V/32)] per task), beam_util.cu:198-220:
+ *     presence_penalty != 0 ? l[t] -= presence_penalty : l[t] = l[t] < 0 ? l[t] * rep : l[t] / rep;
+ *   random iff top_p < 1 || top_k > 0 (batch_generator.h:106); otherwise the argmax of the penalised logits (ties ->
+ *     lowest index, as zl_argmax); defaults (rep 1, presence 0, top_p 1, top_k 0) are plain greedy;
+ *   p = softmax(l / temperature) (softmax.cu:10-30), cum = inclusive sum of p sorted descending (ties in ascending
+ *     index order), P = top_k > 0 ? min(top_p, cum[top_k-1]) : top_p, v = u * P * cum[V-1], pick the first sorted
+ *     position with cum >= v (random_util.cu:83-106);
+ *   u = zl_sample_uniform(seed, draw_counters[task]).
+ * Then sets the pick's seen bit, advances draw_counters[task] and writes out[b].  The logits are not modified.
+ * Requires temperature > 0, 0 <= top_p <= 1, 0 <= top_k < V (random_util.cu:121-122; checked by
+ * zl_llama_set_sampling, not here).  Computes in fp32 / fp64 on the fp32 logits; V <= 327680. */
+typedef struct zl_sample_params {
+    float temperature, top_p, repetition_penalty, presence_penalty;
+    int top_k;
+    uint64_t seed;
+} zl_sample_params_t;
+size_t zl_sample_workspace_bytes(int T, int V);
+int zl_sample(const float* logits, int T, int V, const int32_t* row_task, const zl_sample_params_t* params,
+              uint32_t* seen_bits, uint32_t* draw_counters, int32_t* out, void* workspace, size_t workspace_bytes,
+              int pdl, zl_stream_t stream);
+/* host: the u in (0, 1] the kernel draws: Philox4x32-10 with key = seed, counter = {draw_index, 0, 0, 0},
+ * u = ((w0 >> 8) + 1) * 2^-24.  (The reference draws with curand; the stream differs, the distribution does not.) */
+float zl_sample_uniform(uint64_t seed, uint64_t draw_index);
 /* synthetic-checkpoint generators (bench / tests): counter-based hash RNG, reproducible per seed. */
 int zl_fill_random_u32(uint32_t* p, size_t n, uint64_t seed, zl_stream_t stream);
 int zl_fill_const_u32(uint32_t* p, size_t n, uint32_t value, zl_stream_t stream);
@@ -396,6 +421,14 @@ int zl_llama_sync(zl_llama_t* m);
  * overwrites the next-token / logits row 0 outputs, which zl_llama_step_device consumes before it returns. */
 int zl_llama_prefill(zl_llama_t* m, int task, const int32_t* tokens_host, int n, int pos0, int32_t* next_token_host,
                      float* logits_host);
+/* Sampling state of one task (SearchTask's temperature / top_p / top_k / repetition_penalty / presence_penalty /
+ * seed, batch_generator.cpp:1639-1692): validates host_params, copies them to the device and clears the task's seen
+ * set and draw counter.  Steps whose batch holds a task with such state pick with zl_sample instead of zl_argmax (a
+ * graph of its own; later parameter changes reuse it).  tp_size > 1: ZL_ERR_UNSUPPORTED (top-p over vocabulary shards
+ * needs a global select). */
+int zl_llama_set_sampling(zl_llama_t* m, int task, const zl_sample_params_t* host_params);
+/* back to plain greedy picks for this task. */
+int zl_llama_clear_sampling(zl_llama_t* m, int task);
 zl_stream_t zl_llama_stream(zl_llama_t* m);
 /* bytes the step must read from HBM per rank (weights + lm_head + norms), kernel launches per step. */
 int zl_llama_stats(zl_llama_t* m, int B, double* weight_bytes, int* kernels_per_step);

@@ -38,6 +38,14 @@ class LlamaConfig(ctypes.Structure):
     ]
 
 
+class SampleParams(ctypes.Structure):
+    """zl_sample_params_t"""
+    _fields_ = [
+        ("temperature", ctypes.c_float), ("top_p", ctypes.c_float), ("repetition_penalty", ctypes.c_float),
+        ("presence_penalty", ctypes.c_float), ("top_k", ctypes.c_int), ("seed", ctypes.c_uint64),
+    ]
+
+
 class W4FusedArgs(ctypes.Structure):
     """zl_w4_fused_args_t"""
     _fields_ = [
@@ -86,6 +94,7 @@ def parse_header(path=HEADER):
     src = re.sub(r"//[^\n]*", " ", src)
     src = re.sub(r"typedef struct zl_llama_config \{.*?\} zl_llama_config_t;", " ", src, flags=re.S)
     src = re.sub(r"typedef struct zl_w4_fused_args \{.*?\} zl_w4_fused_args_t;", " ", src, flags=re.S)
+    src = re.sub(r"typedef struct zl_sample_params \{.*?\} zl_sample_params_t;", " ", src, flags=re.S)
     protos = {}
     for m in re.finditer(r"([A-Za-z_][\w \*]*?)\b(zl_\w+)\s*\(([^;{}]*?)\)\s*;", src):
         ret, name, args = m.group(1).strip(), m.group(2), m.group(3).strip()

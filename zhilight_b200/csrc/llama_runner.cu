@@ -94,7 +94,7 @@ struct zl_llama {
     int vshard = 0;                       // vocabulary rows of lm_head held by this rank
     void* cand = nullptr;                 // [B] {float value, int index} local argmax candidates
     void* cand_all = nullptr;             // [tp][B] gathered candidates
-    std::map<long long, cudaGraphExec_t> graphs;   // key = B * 2^32 + attention length bucket
+    std::map<long long, cudaGraphExec_t> graphs;   // key = B * 2^33 + sampling * 2^32 + attention length bucket
     int cur_max_len = 0;                            // host-side upper bound of buf_lens (positions + 1)
     double weight_bytes = 0;
     int kernels_per_step = 0;
@@ -109,6 +109,12 @@ struct zl_llama {
     int32_t* d_tb = nullptr;      // token -> task map of the chunk being prefilled
     const int32_t* cur_tb = nullptr;   // token -> task map of the launch sequence being enqueued (d_iota at decode)
     int8_t* d_mask = nullptr;     // (chunk, max_seq) causal mask of the chunk
+    // sampling (zl_llama_set_sampling): per-task parameters, seen-token bits and draw counters on the device, read by
+    // the graph at replay time; a host flag per task selects the zl_sample graph for batches that hold such a task
+    zl_sample_params_t* d_sparams = nullptr;   // (max_batch)
+    uint32_t* d_seen = nullptr;                // (max_batch, ceil(vshard / 32))
+    uint32_t* d_draws = nullptr;               // (max_batch)
+    std::vector<char> sampling;                // (max_batch) task has non-default sampling state
 };
 
 namespace {
@@ -553,6 +559,18 @@ int finalize_globals(zl_llama* m) {
     return ZL_OK;
 }
 
+// the parameters of a task without sampling state: zl_sample then picks exactly what zl_argmax picks
+constexpr zl_sample_params_t kGreedyParams = {1.0f, 1.0f, 1.0f, 0.0f, 0, 0};
+
+// stream-ordered: parameters to the device, seen set and draw counter cleared
+int write_sampling(zl_llama* m, int task, const zl_sample_params_t& p) {
+    const size_t words = (size_t)(m->vshard + 31) / 32;
+    ZL_CHECK_CUDA(cudaMemcpyAsync(m->d_sparams + task, &p, sizeof(p), cudaMemcpyHostToDevice, m->stream));
+    ZL_CHECK_CUDA(cudaMemsetAsync(m->d_seen + task * words, 0, words * sizeof(uint32_t), m->stream));
+    ZL_CHECK_CUDA(cudaMemsetAsync(m->d_draws + task, 0, sizeof(uint32_t), m->stream));
+    return ZL_OK;
+}
+
 int alloc_runtime(zl_llama* m) {
     const auto& c = m->cfg;
     const int B = c.max_batch, D = c.dim_model, d = c.dim_head;
@@ -608,6 +626,11 @@ int alloc_runtime(zl_llama* m) {
     m->attn_ws_bytes = zl_decode_attention_workspace_bytes(T, 1, m->hq, d, c.max_seq);
     RCHECK(dmalloc(&m->attn_ws, m->attn_ws_bytes));
     RCHECK(dmalloc(&m->argmax_ws, zl_argmax_workspace_bytes(B)));
+    RCHECK(dmalloc((void**)&m->d_sparams, sizeof(zl_sample_params_t) * B));
+    RCHECK(dmalloc((void**)&m->d_seen, sizeof(uint32_t) * B * (size_t)((m->vshard + 31) / 32)));
+    RCHECK(dmalloc((void**)&m->d_draws, sizeof(uint32_t) * B));
+    m->sampling.assign(B, 0);
+    for (int t = 0; t < B; ++t) RCHECK(write_sampling(m, t, kGreedyParams));
     ZL_CHECK_CUDA(cudaMallocHost((void**)&m->h_stage, sizeof(int32_t) * (4 * B + 4 + T)));
     ZL_CHECK_CUDA(cudaMallocHost((void**)&m->h_ring, sizeof(int32_t) * zl_llama::kStageSlots * 2 * B));
     for (int i = 0; i < zl_llama::kStageSlots; ++i)
@@ -864,6 +887,14 @@ int prefill_layers_dual(zl_llama* m, const PrefillChunk& pf) {
     return ZL_OK;
 }
 
+// does the launch sequence for decode tasks 0..n_tasks-1 (or the prefilled task) pick with zl_sample?
+bool step_samples(const zl_llama* m, int n_tasks, const PrefillChunk* pf) {
+    if (pf) return m->sampling[pf->task] != 0;
+    for (int t = 0; t < n_tasks; ++t)
+        if (m->sampling[t]) return true;
+    return false;
+}
+
 int enqueue_step(zl_llama* m, int n_tasks, int len_bucket, const PrefillChunk* pf = nullptr) {
     const auto& c = m->cfg;
     const int B = pf ? pf->n : n_tasks;   // rows (tokens) of every activation matrix in this launch sequence
@@ -1024,7 +1055,11 @@ int enqueue_step(zl_llama* m, int n_tasks, int len_bucket, const PrefillChunk* p
     // vocab-parallel lm_head (embedding.cu:353-392): each rank owns vshard rows
     if (!(skip & 32))
         RCHECK(zl_dense_gemm_skinny(m->xn, D, m->lm_head, nullptr, m->logits, HB, m->vshard, D, dt, ZL_F32, P(64), st));
-    if (!tp) {
+    if (step_samples(m, n_tasks, pf)) {
+        // row 0 of a prefill belongs to pf->task: d_iota[task] == task
+        RCHECK(zl_sample(m->logits, HB, m->vshard, pf ? m->d_iota + pf->task : m->d_iota, m->d_sparams, m->d_seen,
+                         m->d_draws, m->d_next, nullptr, 0, P(128), st));
+    } else if (!tp) {
         RCHECK(zl_argmax(m->logits, m->d_next, HB, m->vshard, m->argmax_ws, zl_argmax_workspace_bytes(HB), P(128), st));
     } else {
         // instead of all-gathering (B, V) logits, exchange one {value, index} candidate per token
@@ -1047,7 +1082,8 @@ int len_bucket_of(const zl_llama* m, int max_len) {
 int run_step(zl_llama* m, int B) {
     const int bucket = len_bucket_of(m, m->cur_max_len);
     if (!m->cfg.use_graph) return enqueue_step(m, B, bucket);
-    const long long key = ((long long)B << 32) | (unsigned)bucket;
+    // sampling steps have a graph of their own: batches without a sampling task replay exactly the greedy graph
+    const long long key = ((long long)B << 33) | ((long long)step_samples(m, B, nullptr) << 32) | (unsigned)bucket;
     auto it = m->graphs.find(key);
     if (it == m->graphs.end()) {
         cudaGraph_t graph = nullptr;
@@ -1135,7 +1171,8 @@ extern "C" void zl_llama_destroy(zl_llama_t* m) {
     }
     for (void* p : {m->emb, m->lm_head_tied ? nullptr : m->lm_head, m->ln_f, m->h, m->xn, m->qkv, m->q, m->ao, m->act,
                     m->pend, m->gu, (void*)m->logits, (void*)m->cosb, (void*)m->sinb, (void*)m->d_tokens,
-                    m->h2, (void*)m->d_pos, (void*)m->d_lens, (void*)m->d_next, (void*)m->d_iota, m->attn_ws, m->argmax_ws, (void*)m->d_tb, (void*)m->d_mask, m->xq, (void*)m->xs})
+                    m->h2, (void*)m->d_pos, (void*)m->d_lens, (void*)m->d_next, (void*)m->d_iota, m->attn_ws, m->argmax_ws, (void*)m->d_tb, (void*)m->d_mask, m->xq, (void*)m->xs,
+                    (void*)m->d_sparams, (void*)m->d_seen, (void*)m->d_draws})
         if (p) cudaFree(p);
     if (m->reduce_stream) {
         cudaStreamSynchronize(m->reduce_stream);
@@ -1457,6 +1494,44 @@ extern "C" int zl_llama_prefill(zl_llama_t* m, int task, const int32_t* tokens_h
     ZL_CHECK_CUDA(cudaStreamSynchronize(m->stream));
     *next_token_host = m->h_stage[3 * m->cfg.max_batch];
     if (pos0 + n > m->cur_max_len) m->cur_max_len = pos0 + n;
+    return ZL_OK;
+}
+
+extern "C" int zl_llama_set_sampling(zl_llama_t* m, int task, const zl_sample_params_t* host_params) {
+    ZL_CHECK_ARG(m && host_params);
+    if (m->cfg.tp_size > 1) {
+        zl_set_last_error(__FILE__, __LINE__,
+                          "unsupported: sampling with tp_size > 1 (top-p over vocabulary shards needs a global select)");
+        return ZL_ERR_UNSUPPORTED;
+    }
+    if (!m->finalized) {
+        zl_set_last_error(__FILE__, __LINE__, "model not finalized");
+        return ZL_ERR_STATE;
+    }
+    ZL_CHECK_ARG(task >= 0 && task < m->cfg.max_batch);
+    const zl_sample_params_t& p = *host_params;
+    // random_util.cu:121-122
+    ZL_CHECK_ARG(p.temperature > 0.0f && p.temperature <= 3.0e38f);
+    ZL_CHECK_ARG(p.top_p >= 0.0f && p.top_p <= 1.0f);
+    ZL_CHECK_ARG(p.top_k >= 0 && p.top_k < m->cfg.vocab_size);
+    ZL_CHECK_ARG(p.repetition_penalty > 0.0f && p.repetition_penalty <= 3.0e38f);
+    ZL_CHECK_ARG(p.presence_penalty == p.presence_penalty && p.presence_penalty >= -3.0e38f &&
+                 p.presence_penalty <= 3.0e38f);
+    RCHECK(write_sampling(m, task, p));
+    m->sampling[task] = 1;
+    return ZL_OK;
+}
+
+extern "C" int zl_llama_clear_sampling(zl_llama_t* m, int task) {
+    ZL_CHECK_ARG(m);
+    if (!m->finalized) {
+        zl_set_last_error(__FILE__, __LINE__, "model not finalized");
+        return ZL_ERR_STATE;
+    }
+    ZL_CHECK_ARG(task >= 0 && task < m->cfg.max_batch);
+    if (m->cfg.tp_size > 1) return ZL_OK;   // never set
+    RCHECK(write_sampling(m, task, kGreedyParams));
+    m->sampling[task] = 0;
     return ZL_OK;
 }
 

@@ -53,5 +53,6 @@ cudaError_t launch_w4_tc(const W4Params& p, bool pdl, cudaStream_t stream);
 bool w4_tc_supports(int mc, int N, int K);
 cudaError_t prepare_w4_tc();
 cudaError_t prepare_w8_tc();   // w8_tc.cu
+cudaError_t prepare_sample();  // sample.cu
 
 }  // namespace zl

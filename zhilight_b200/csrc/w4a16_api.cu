@@ -21,6 +21,7 @@ extern "C" int zl_prepare(void) {
     ZL_CHECK_CUDA(prepare_w4_v3());
     ZL_CHECK_CUDA(prepare_w4_tc());
     ZL_CHECK_CUDA(prepare_w8_tc());
+    ZL_CHECK_CUDA(prepare_sample());
     return ZL_OK;
 }
 

@@ -123,6 +123,19 @@ class LlamaDecoder:
         _lib.check(self.lib.zl_llama_get_logits(self.h, out.ctypes.data_as(ctypes.c_void_p), b))
         return out
 
+    def set_sampling(self, task, temperature=1.0, top_p=1.0, top_k=0, repetition_penalty=1.0, presence_penalty=0.0,
+                     seed=0):
+        """Seeded top-k / top-p sampling with repetition / presence penalties for `task` (SearchTask fields of the
+        reference): clears the task's seen set and draw counter.  Picks of steps whose batch holds the task come from
+        zl_sample; raises ZLError(-2) with tp_size > 1."""
+        p = _lib.SampleParams(float(temperature), float(top_p), float(repetition_penalty), float(presence_penalty),
+                              int(top_k), int(seed) & 0xFFFFFFFFFFFFFFFF)
+        _lib.check(self.lib.zl_llama_set_sampling(self.h, int(task), ctypes.byref(p)))
+
+    def clear_sampling(self, task):
+        """Back to plain greedy picks for `task`."""
+        _lib.check(self.lib.zl_llama_clear_sampling(self.h, int(task)))
+
     def step_device(self, b):
         _lib.check(self.lib.zl_llama_step_device(self.h, b))
 

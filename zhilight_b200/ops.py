@@ -392,3 +392,48 @@ def argmax(logits):
     ws = torch.empty(nb, dtype=torch.uint8, device=logits.device)
     _lib.call("zl_argmax", _p(logits), _p(out), t, v, _p(ws), nb, 0, _stream())
     return out
+
+
+def sample_params(tasks, device, vocab):
+    """zl_sample_params_t records on `device` (a uint8 tensor) from a list of dicts with the keys of
+    LlamaDecoder.set_sampling (temperature, top_p, top_k, repetition_penalty, presence_penalty, seed), validated as
+    random_util.cu:121-122 asserts (temperature > 0, 0 <= top_p <= 1, 0 <= top_k < vocab)."""
+    recs = (_lib.SampleParams * len(tasks))()
+    for i, t in enumerate(tasks):
+        r = recs[i]
+        r.temperature = float(t.get("temperature", 1.0))
+        r.top_p = float(t.get("top_p", 1.0))
+        r.top_k = int(t.get("top_k", 0))
+        r.repetition_penalty = float(t.get("repetition_penalty", 1.0))
+        r.presence_penalty = float(t.get("presence_penalty", 0.0))
+        r.seed = int(t.get("seed", 0)) & 0xFFFFFFFFFFFFFFFF
+        if not (r.temperature > 0 and 0 <= r.top_p <= 1 and 0 <= r.top_k < vocab and r.repetition_penalty > 0):
+            raise _lib.ZLError(-1, "invalid sampling parameters %r" % (t,))
+    raw = bytes(recs)
+    return torch.frombuffer(bytearray(raw), dtype=torch.uint8).to(device)
+
+
+def sample(logits, params, seen_bits, draw_counters, row_task=None):
+    """zl_sample: one pick per row of fp32 logits (T, V).  params: sample_params(...) of the tasks; seen_bits: int32
+    (tasks, ceil(V/32)) seen-token bits; draw_counters: int32 (tasks); row_task: int32 (T) task of each row (default
+    row i -> task i).  Updates seen_bits and draw_counters in place like the decode driver; returns int32 (T)."""
+    t, v = logits.shape
+    if row_task is None:
+        row_task = torch.arange(t, dtype=torch.int32, device=logits.device)
+    for x, dt in ((logits, torch.float32), (seen_bits, torch.int32), (draw_counters, torch.int32), (row_task, torch.int32)):
+        if x.dtype != dt:
+            raise _lib.ZLError(-1, "sample: expected %s, got %s" % (dt, x.dtype))
+    if seen_bits.shape[-1] != (v + 31) // 32:
+        raise _lib.ZLError(-1, "seen_bits must hold ceil(V/32) words per task")
+    out = torch.empty(t, dtype=torch.int32, device=logits.device)
+    nb = _lib.load().zl_sample_workspace_bytes(t, v)
+    ws = torch.empty(max(nb, 1), dtype=torch.uint8, device=logits.device)
+    _lib.call("zl_sample", _p(logits), t, v, _p(row_task), _p(params), _p(seen_bits), _p(draw_counters), _p(out), _p(ws),
+              nb, 0, _stream())
+    return out
+
+
+def sample_uniform(seed, draw_index):
+    """The u in (0, 1] zl_sample draws for (seed, draw_index) (host computation, no GPU needed)."""
+    lib = _lib.load()
+    return float(lib.zl_sample_uniform(int(seed) & 0xFFFFFFFFFFFFFFFF, int(draw_index)))
